@@ -1,5 +1,5 @@
 """Synthetic scene generators for the configs of BASELINE.json (SURVEY.md section 8d) plus a loader for
-the reference's own Sponza geometry (used only by local tests; /root/reference does not exist on the GPU box).
+the reference's own Sponza geometry (tests/golden/ keeps a sample of it for the tests).
 
 All generators are seeded and deterministic; all materials use constant (1x1) textures, i.e. factors only
 (the reference's own fallback for missing maps, SRC/Utils/ModelLoader.cs:877-885).
@@ -431,8 +431,9 @@ def texturize(scene, size=512, count=8, seed=11):
     return scene
 
 
-# --------------------------------------------------------------------------- real Sponza (local only)
-REFERENCE_SPONZA = "/root/reference/IDKEngine/Resource/Models/SponzaCompressed/Sponza.gltf"
+# --------------------------------------------------------------------------- real Sponza (IDKEngine's Resource/Models/SponzaCompressed/Sponza.gltf)
+SPONZA_PLACEMENT = (1.815, 0.0, (0.0, -1.0, 0.0))          # trs_matrix(scale, yaw, translation) of SRC/Application.cs:448
+SPONZA_CAMERA = dict(position=(7.63, 2.71, 0.8), view_dir=tuple(view_dir_from_angles(360.0 - 165.4, 90.0 - 7.4)), fov_y_deg=102.0)
 
 
 def load_gltf_geometry(path):
@@ -478,10 +479,11 @@ def load_gltf_geometry(path):
     return g, pos, nrm, uv, idx, tri_mesh, mesh_mat
 
 
-def sponza_reference(threads=None):
-    """Config 2 with the reference's real Sponza.bin geometry (262,267 triangles). Materials from glTF factors with
-    metallic=0, roughness=0.8 (SURVEY 8d 'constant-texture semantics'); emissive biases per SRC/Application.cs:449-457."""
-    g, pos, nrm, uv, idx, tri_mesh, mesh_mat = load_gltf_geometry(REFERENCE_SPONZA)
+def sponza_reference(path, threads=None):
+    """Config 2 with the reference's real Sponza.bin geometry (262,267 triangles), read from the Sponza.gltf at `path`.
+    Materials from glTF factors with metallic=0, roughness=0.8 (SURVEY 8d 'constant-texture semantics'); emissive biases
+    per SRC/Application.cs:449-457."""
+    g, pos, nrm, uv, idx, tri_mesh, mesh_mat = load_gltf_geometry(path)
     gm = g.get("materials", [{}])
     mats = gt.default_material(len(gm))
     for k, m in enumerate(gm):
@@ -501,10 +503,9 @@ def sponza_reference(threads=None):
     normals = None if any(n is None for n in nrm) else np.concatenate(nrm)
     model = Model(np.concatenate(pos), np.concatenate(idx), np.concatenate(tri_mesh), normals=normals,
                   texcoords=np.concatenate(uv), meshes=meshes, materials=mats,
-                  model_matrix=trs_matrix(1.815, 0.0, (0.0, -1.0, 0.0)), name="sponza")
+                  model_matrix=trs_matrix(*SPONZA_PLACEMENT), name="sponza")
     scene = Scene().add(model, threads=threads)
-    cam = dict(position=(7.63, 2.71, 0.8), view_dir=tuple(view_dir_from_angles(360.0 - 165.4, 90.0 - 7.4)), fov_y_deg=102.0)
-    return scene, cam
+    return scene, dict(SPONZA_CAMERA)
 
 
 def camera_frame(cam, width, height):

@@ -14,7 +14,7 @@ LIBORACLE = os.path.join(ORACLE_DIR, "liboracle.so")
 
 def build(force=False, verbose=False):
     src = os.path.join(ORACLE_DIR, "oracle.cpp")
-    deps = [src, os.path.join(ORACLE_DIR, "oracle_vxgi.inc")] + [os.path.join(ORACLE_DIR, "..", "include", f) for f in ("idkpt.h", "idkvx.h", "idk_gpu_types.h")]
+    deps = [src] + [os.path.join(ORACLE_DIR, f) for f in ("oracle_vxgi.inc", "oracle_post.inc")] + [os.path.join(ORACLE_DIR, "..", "include", f) for f in ("idkpt.h", "idkvx.h", "idk_gpu_types.h")]
     if not force and os.path.exists(LIBORACLE) and all(os.path.getmtime(d) <= os.path.getmtime(LIBORACLE) for d in deps):
         return LIBORACLE
     cmd = ["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-shared", "-pthread",
