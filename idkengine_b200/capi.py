@@ -96,7 +96,18 @@ EXPORTS = [
     "idkpt_read_wavefront_rays", "idkpt_trace_rays", "idkpt_trace_rays_any", "idkpt_shadows_ray_traced",
     "idkpt_set_skinning_data", "idkpt_skin_vertices", "idkpt_blas_refit", "idkpt_read_range", "idkpt_post_process", "idkpt_ldr_device_ptr", "idkpt_abi_version",
     "idkpt_denoise", "idkpt_denoise_device_ptrs", "idkpt_denoise_import_output", "idkpt_tlas_build",
+    "idkpt_blas_default_build_settings", "idkpt_blas_build", "idkpt_blas_build_read", "idkpt_blas_build_phase_ms",
 ]
+
+
+class IdkPtBlasBuildSettings(ctypes.Structure):
+    _fields_ = [("StopSplittingThreshold", c_i32), ("MaxLeafTriangleCount", c_i32), ("TriangleCost", c_f),
+                ("StackOptThreshold", c_i32), ("StackOptSahIncreaseAcceptance", c_f), ("SplitFactor", c_f), ("DoPreSplit", c_i32)]
+
+
+class IdkPtBlasBuildInfo(ctypes.Structure):
+    _fields_ = [("NodeCount", c_u32), ("TriangleCount", c_u32), ("FragmentCount", c_u32), ("RequiredStackSize", c_i32),
+                ("SahBits", c_u64)]
 
 
 class IdkPtDenoiseSettings(ctypes.Structure):
@@ -297,6 +308,14 @@ def load(path=None):
     L.idkpt_denoise_device_ptrs.argtypes = [c_vp, P(c_vp), P(c_vp), P(c_vp), P(c_vp), P(c_u64)]
     L.idkpt_denoise_import_output.restype = c_i32
     L.idkpt_denoise_import_output.argtypes = [c_vp]
+    L.idkpt_blas_default_build_settings.restype = None
+    L.idkpt_blas_default_build_settings.argtypes = [P(IdkPtBlasBuildSettings)]
+    L.idkpt_blas_build.restype = c_i32
+    L.idkpt_blas_build.argtypes = [c_vp, c_vp, c_u64, c_vp, c_u64, c_vp, c_u32, P(IdkPtBlasBuildSettings), c_vp, P(c_f)]
+    L.idkpt_blas_build_read.restype = c_i32
+    L.idkpt_blas_build_read.argtypes = [c_vp, c_u32, c_vp, c_vp]
+    L.idkpt_blas_build_phase_ms.restype = c_i32
+    L.idkpt_blas_build_phase_ms.argtypes = [c_vp, P(c_f), c_i32]
     L.idkpt_abi_version.restype = c_u32
     L.idkpt_abi_version.argtypes = []
     if path == _build.LIBIDKPT:

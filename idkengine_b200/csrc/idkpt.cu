@@ -16,6 +16,7 @@
 #include "idk_shadows.cuh"
 #include "idk_dynamic.cuh"
 #include "idk_post.cuh"
+#include "idk_blas_build.cuh"
 #include "idk_textures_host.h"
 
 #define IDKPT_ABI_VERSION 4u   // 2: IdkPtSceneDesc gained Textures / TextureCount; 3: IdkPtStats gained CompactMs / AccumulateMs, host-buffer registration;
@@ -139,6 +140,15 @@ struct IdkPtCtx {
     cudaEvent_t snapDone = nullptr, copyDone = nullptr;
     DevBuf presentSnap;
     bool copyPending = false;
+
+    // device BLAS build (idkpt_blas_build): its own stream and buffers, the results of the last build
+    struct BlasBuild {
+        cudaStream_t stream = nullptr;
+        DevBuf buf[48];
+        std::vector<IdkPtBlasBuildInfo> infos;
+        std::vector<int> nodeBase, fragOffset;
+        float phaseMs[6] = {};
+    } bb;
 };
 
 #define CK(call)                                                                                   \
@@ -597,6 +607,8 @@ IDKPT_API void idkpt_destroy(IdkPtCtx* ctx) {
     if (ctx->snapDone) cudaEventDestroy(ctx->snapDone);
     if (ctx->copyDone) cudaEventDestroy(ctx->copyDone);
     release(ctx->presentSnap);
+    for (DevBuf& b : ctx->bb.buf) release(b);
+    if (ctx->bb.stream) cudaStreamDestroy(ctx->bb.stream);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
 }
@@ -1987,6 +1999,333 @@ static int trace_rays_impl(IdkPtCtx* ctx, const IdkPtRay* rays, uint64_t count, 
     if (e0) cudaEventDestroy(e0);
     if (e1) cudaEventDestroy(e1);
     return rc;
+}
+
+
+// ---- device BLAS build (idk_blas_build.cuh) ----
+enum BbBuf {
+    BB_POS, BB_TRIS, BB_ITEMSTART, BB_TRIOFF, BB_PRESPLIT, BB_PRIO, BB_TOTALPRIO, BB_GBOX, BB_SPLITCOUNT, BB_ITEMBLAS,
+    BB_BLASOFF, BB_BOUNDS, BB_FRAGTRI, BB_FRAGBLAS, BB_KEYS, BB_KEYS2, BB_VALS, BB_SORTED0, BB_SORTED1, BB_SORTED2,
+    BB_TABLE, BB_AUX, BB_R0, BB_R1, BB_R2, BB_STACK, BB_NODES, BB_OUT, BB_DEPTH, BB_PARENT, BB_RSTART, BB_RCOUNT,
+    BB_FRAGOFF, BB_FRAGCOUNT, BB_NODEBASE, BB_TASKS0, BB_TASKS1, BB_SMALL, BB_COUNTERS, BB_PERBLAS, BB_NODEI0, BB_NODEI1,
+    BB_NODEI2, BB_NODEI3, BB_NODED0, BB_NODED1, BB_TRIOUT, BB_TEMP, BB_COUNT
+};
+static_assert(BB_COUNT <= 48, "IdkPtCtx::BlasBuild::buf");
+
+__global__ void k_bb_gather_offsets(const long long* offset, const int* itemStart, int blasCount, long long* out) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b <= blasCount) out[b] = offset[itemStart[b]];
+}
+
+__global__ void k_bb_init_roots(idkbb::SplitArgs a, const int* fragCount, int blasCount) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= blasCount) return;
+    const int n = fragCount[b];
+    idkbb::createChild(a, a.nodeBase[b], 1, -1, 0, n, 0);
+    idkbb::pushTask(a, {b, 1, 2, 0}, n);
+}
+
+static int bits_for(uint64_t v) { int b = 0; while (v) { b++; v >>= 1; } return b; }
+
+IDKPT_API void idkpt_blas_default_build_settings(IdkPtBlasBuildSettings* s) {
+    if (!s) return;
+    s->StopSplittingThreshold = 1;
+    s->MaxLeafTriangleCount = 2;
+    s->TriangleCost = 1.1f;
+    s->StackOptThreshold = 16;
+    s->StackOptSahIncreaseAcceptance = 0.0009745f;
+    s->SplitFactor = 0.3f;
+    s->DoPreSplit = 1;
+}
+
+static inline float bb_half_area(const float mn[3], const float mx[3]) {
+    const float sx = mx[0] - mn[0], sy = mx[1] - mn[1], sz = mx[2] - mn[2];
+    return fmaf(sx + sy, sz, sx * sy);
+}
+
+IDKPT_API int idkpt_blas_build(IdkPtCtx* ctx, const PackedVec3* positions, uint64_t positionCount, const GpuBlasTriangle* triangles,
+                               uint64_t triangleCount, const IdkPtBlasBuildDesc* descs, uint32_t blasCount,
+                               const IdkPtBlasBuildSettings* settings, IdkPtBlasBuildInfo* infosOut, float* kernelMs) {
+    if (!ctx) return IDKPT_ERR_INVALID_ARGUMENT;
+    if (kernelMs) *kernelMs = 0.0f;
+    auto& bb = ctx->bb;
+    bb.infos.clear();
+    bb.nodeBase.clear();
+    bb.fragOffset.clear();
+    if (blasCount == 0) return IDKPT_OK;
+    if (!descs || !infosOut || (!positions && positionCount) || (!triangles && triangleCount))
+        return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build: null argument");
+    if (blasCount > 65535) return fail(ctx, IDKPT_ERR_UNSUPPORTED, "idkpt_blas_build: more than 65535 BLASes in one call");
+    IdkPtBlasBuildSettings st;
+    if (settings) st = *settings; else idkpt_blas_default_build_settings(&st);
+
+    // ---- validation (host arrays, before any device work)
+    for (uint64_t i = 0; i < positionCount; i++)
+        if (!std::isfinite(positions[i].x) || !std::isfinite(positions[i].y) || !std::isfinite(positions[i].z))
+            return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build: non-finite vertex position");
+    uint64_t items = 0;
+    for (uint32_t b = 0; b < blasCount; b++) {
+        const IdkPtBlasBuildDesc& d = descs[b];
+        if (d.TriangleCount == 0) return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build: empty BLAS");
+        if ((uint64_t)d.TriangleOffset + d.TriangleCount > triangleCount) return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build: BLAS triangle range outside the triangle array");
+        if (d.TriangleCount >= (uint32_t)idkbb::MAX_FRAGMENTS) return fail(ctx, IDKPT_ERR_UNSUPPORTED, "idkpt_blas_build: a BLAS of 2^24 or more fragments");
+        float mn[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, mx[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+        for (uint32_t t = d.TriangleOffset; t < d.TriangleOffset + d.TriangleCount; t++) {
+            const int32_t id[3] = {triangles[t].X, triangles[t].Y, triangles[t].Z};
+            for (int v = 0; v < 3; v++) {
+                if (id[v] < 0 || (uint64_t)id[v] >= positionCount) return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build: vertex index outside the position array");
+                const float p[3] = {positions[id[v]].x, positions[id[v]].y, positions[id[v]].z};
+                for (int k = 0; k < 3; k++) { mn[k] = std::min(mn[k], p[k]); mx[k] = std::max(mx[k], p[k]); }
+            }
+        }
+        if (!std::isfinite(bb_half_area(mn, mx))) return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build: BLAS bounding box with a non-finite half-area");
+        items += d.TriangleCount;
+    }
+    if (items >= (1ull << 31)) return fail(ctx, IDKPT_ERR_UNSUPPORTED, "idkpt_blas_build: 2^31 or more triangles in one call");
+    const int B = (int)blasCount, W = (int)items;
+    std::vector<int> itemStart(B + 1), triOff(B), presplit(B);
+    for (int b = 0; b < B; b++) {
+        itemStart[b + 1] = itemStart[b] + (int)descs[b].TriangleCount;
+        triOff[b] = (int)descs[b].TriangleOffset;
+        presplit[b] = st.DoPreSplit && !descs[b].IsRefittable;
+    }
+
+    CK(cudaSetDevice(ctx->device));
+    if (!bb.stream) CK(cudaStreamCreateWithFlags(&bb.stream, cudaStreamNonBlocking));
+    cudaStream_t s = bb.stream;
+    DevBuf* buf = bb.buf;
+    auto need = [&](int id, size_t bytes) { return ensure(buf[id], std::max<size_t>(bytes, 16)); };
+#define BB_NEED(id, bytes) do { if (need(id, bytes) != cudaSuccess) return fail(ctx, IDKPT_ERR_OUT_OF_MEMORY, "idkpt_blas_build: device allocation failed"); } while (0)
+#define BB_P(id, T) ((T*)buf[id].p)
+    size_t tempBytes = 0;
+    auto temp = [&](size_t bytes) -> cudaError_t { tempBytes = bytes; return need(BB_TEMP, bytes); };
+
+    cudaEvent_t ev[7];
+    for (int i = 0; i < 7; i++) CK(cudaEventCreate(&ev[i]));
+    struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 7; i++) cudaEventDestroy(e[i]); } } evGuard{ev};
+
+    // ---- pre-splitting
+    BB_NEED(BB_POS, positionCount * 12); BB_NEED(BB_TRIS, triangleCount * 16);
+    BB_NEED(BB_ITEMSTART, (B + 1) * 4); BB_NEED(BB_TRIOFF, B * 4); BB_NEED(BB_PRESPLIT, B * 4);
+    BB_NEED(BB_PRIO, (size_t)W * 4); BB_NEED(BB_TOTALPRIO, B * 4); BB_NEED(BB_GBOX, B * sizeof(idkbb::Box));
+    BB_NEED(BB_SPLITCOUNT, ((size_t)W + 1) * 8); BB_NEED(BB_ITEMBLAS, (size_t)W * 4); BB_NEED(BB_BLASOFF, (B + 1) * 8);
+    if (positionCount) CK(cudaMemcpyAsync(buf[BB_POS].p, positions, positionCount * 12, cudaMemcpyHostToDevice, s));
+    if (triangleCount) CK(cudaMemcpyAsync(buf[BB_TRIS].p, triangles, triangleCount * 16, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(buf[BB_ITEMSTART].p, itemStart.data(), (B + 1) * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(buf[BB_TRIOFF].p, triOff.data(), B * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(buf[BB_PRESPLIT].p, presplit.data(), B * 4, cudaMemcpyHostToDevice, s));
+    cudaEventRecord(ev[0], s);
+    idkbb::PreArgs pa;
+    pa.pos = BB_P(BB_POS, float); pa.tris = BB_P(BB_TRIS, int4); pa.blasItemStart = BB_P(BB_ITEMSTART, int);
+    pa.blasTriOffset = BB_P(BB_TRIOFF, int); pa.blasPresplit = BB_P(BB_PRESPLIT, int); pa.itemCount = W; pa.blasCount = B;
+    pa.prio = BB_P(BB_PRIO, float); pa.totalPrio = BB_P(BB_TOTALPRIO, float); pa.globalBox = BB_P(BB_GBOX, idkbb::Box);
+    pa.splitCount = BB_P(BB_SPLITCOUNT, long long); pa.itemBlas = BB_P(BB_ITEMBLAS, int); pa.splitFactor = st.SplitFactor;
+    idkbb::k_item_prepare<<<(W + 255) / 256, 256, 0, s>>>(pa);
+    idkbb::k_total_priority<<<(B + 127) / 128, 128, 0, s>>>(pa);
+    idkbb::k_global_box<<<B, idkbb::NT, 0, s>>>(pa);
+    idkbb::k_split_counts<<<(W + 256) / 256, 256, 0, s>>>(pa);
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tempBytes, pa.splitCount, pa.splitCount, W + 1, s));
+    CK(temp(tempBytes));
+    CK(cub::DeviceScan::ExclusiveSum(buf[BB_TEMP].p, tempBytes, pa.splitCount, pa.splitCount, W + 1, s));
+    k_bb_gather_offsets<<<(B + 128) / 128, 128, 0, s>>>(pa.splitCount, pa.blasItemStart, B, BB_P(BB_BLASOFF, long long));
+    std::vector<long long> blasOff(B + 1);
+    CK(cudaMemcpyAsync(blasOff.data(), buf[BB_BLASOFF].p, (B + 1) * 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    std::vector<int> fragOff(B), fragCount(B), nodeBase(B + 1);
+    long long nodeSlots = 0;
+    for (int b = 0; b < B; b++) {
+        const long long n = blasOff[b + 1] - blasOff[b];
+        if (n >= idkbb::MAX_FRAGMENTS) return fail(ctx, IDKPT_ERR_UNSUPPORTED, "idkpt_blas_build: a BLAS of 2^24 or more fragments");
+        fragOff[b] = (int)blasOff[b];
+        fragCount[b] = (int)n;
+        nodeBase[b] = (int)nodeSlots;
+        nodeSlots += std::max<long long>(2 * n, 4);
+        if (nodeSlots >= (1ll << 31) || blasOff[b + 1] >= (1ll << 30)) return fail(ctx, IDKPT_ERR_UNSUPPORTED, "idkpt_blas_build: too many fragments in one call");
+    }
+    nodeBase[B] = (int)nodeSlots;
+    const int F = (int)blasOff[B], NS = (int)nodeSlots;
+
+    BB_NEED(BB_BOUNDS, (size_t)F * sizeof(idkbb::Box)); BB_NEED(BB_FRAGTRI, (size_t)F * 4); BB_NEED(BB_FRAGBLAS, (size_t)F * 4);
+    idkbb::FragArgs fa;
+    fa.pos = pa.pos; fa.tris = pa.tris; fa.blasItemStart = pa.blasItemStart; fa.blasTriOffset = pa.blasTriOffset;
+    fa.blasPresplit = pa.blasPresplit; fa.itemBlas = pa.itemBlas; fa.offset = pa.splitCount; fa.globalBox = pa.globalBox;
+    fa.itemCount = W; fa.fragCount = F;
+    fa.bounds = BB_P(BB_BOUNDS, idkbb::Box); fa.fragTri = BB_P(BB_FRAGTRI, int); fa.fragBlas = BB_P(BB_FRAGBLAS, int);
+    idkbb::k_fragments<<<(F + 255) / 256, 256, 0, s>>>(fa);
+    cudaEventRecord(ev[1], s);
+
+    // ---- three stable sorts by centroid key (the BLAS id in the high bits keeps every BLAS in its own range)
+    const size_t keyN = std::max<size_t>(F, NS);
+    BB_NEED(BB_KEYS, keyN * 8); BB_NEED(BB_KEYS2, keyN * 8); BB_NEED(BB_VALS, keyN * 4);
+    BB_NEED(BB_SORTED0, (size_t)F * 4); BB_NEED(BB_SORTED1, (size_t)F * 4); BB_NEED(BB_SORTED2, (size_t)F * 4);
+    unsigned long long *keys = BB_P(BB_KEYS, unsigned long long), *keys2 = BB_P(BB_KEYS2, unsigned long long);
+    int* vals = BB_P(BB_VALS, int);
+    int* sorted[3] = {BB_P(BB_SORTED0, int), BB_P(BB_SORTED1, int), BB_P(BB_SORTED2, int)};
+    const int fragEndBit = 32 + bits_for((uint64_t)(B - 1));
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, tempBytes, keys, keys2, vals, sorted[0], F, 0, fragEndBit, s));
+    CK(temp(tempBytes));
+    for (int axis = 0; axis < 3; axis++) {
+        idkbb::k_sort_keys<<<(F + 255) / 256, 256, 0, s>>>(fa.bounds, fa.fragBlas, F, axis, keys, vals);
+        CK(cub::DeviceRadixSort::SortPairs(buf[BB_TEMP].p, tempBytes, keys, keys2, vals, sorted[axis], F, 0, fragEndBit, s));
+    }
+    cudaEventRecord(ev[2], s);
+
+    // ---- splits: the top of every tree level by level, one block per node; subtrees of <= SMALL fragments one thread each
+    BB_NEED(BB_TABLE, F); BB_NEED(BB_AUX, (size_t)F * 4); BB_NEED(BB_R0, (size_t)F * 4); BB_NEED(BB_R1, (size_t)F * 4);
+    BB_NEED(BB_R2, (size_t)F * 4); BB_NEED(BB_STACK, (size_t)F * 12);
+    BB_NEED(BB_NODES, (size_t)NS * 32); BB_NEED(BB_OUT, (size_t)NS * 32); BB_NEED(BB_DEPTH, (size_t)NS * 4);
+    BB_NEED(BB_PARENT, (size_t)NS * 4); BB_NEED(BB_RSTART, (size_t)NS * 4); BB_NEED(BB_RCOUNT, (size_t)NS * 4);
+    BB_NEED(BB_FRAGOFF, B * 4); BB_NEED(BB_FRAGCOUNT, B * 4); BB_NEED(BB_NODEBASE, (B + 1) * 4);
+    const size_t bigCap = (size_t)F / idkbb::SMALL + 2 * (size_t)B + 16, smallCap = 2 * (size_t)F + 2 * (size_t)B + 16;
+    BB_NEED(BB_TASKS0, bigCap * 16); BB_NEED(BB_TASKS1, bigCap * 16); BB_NEED(BB_SMALL, smallCap * 16); BB_NEED(BB_COUNTERS, 64);
+    CK(cudaMemcpyAsync(buf[BB_FRAGOFF].p, fragOff.data(), B * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(buf[BB_FRAGCOUNT].p, fragCount.data(), B * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(buf[BB_NODEBASE].p, nodeBase.data(), (B + 1) * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(buf[BB_NODES].p, 0, (size_t)NS * 32, s));
+    CK(cudaMemsetAsync(buf[BB_DEPTH].p, 0xFF, (size_t)NS * 4, s));
+    CK(cudaMemsetAsync(buf[BB_COUNTERS].p, 0, 64, s));
+    int* counters = BB_P(BB_COUNTERS, int);     // [0], [1]: big-task counts (ping-pong), [2]: small-task count
+    idkbb::SplitArgs sa;
+    sa.bounds = fa.bounds;
+    for (int i = 0; i < 3; i++) sa.sorted[i] = sorted[i];
+    sa.table = BB_P(BB_TABLE, uint8_t); sa.aux = BB_P(BB_AUX, int);
+    sa.R[0] = BB_P(BB_R0, float); sa.R[1] = BB_P(BB_R1, float); sa.R[2] = BB_P(BB_R2, float);
+    sa.stack = BB_P(BB_STACK, int); sa.nodes = BB_P(BB_NODES, GpuBlasNode);
+    sa.depth = BB_P(BB_DEPTH, int); sa.parent = BB_P(BB_PARENT, int); sa.rangeStart = BB_P(BB_RSTART, int); sa.rangeCount = BB_P(BB_RCOUNT, int);
+    sa.fragOffset = BB_P(BB_FRAGOFF, int); sa.nodeBase = BB_P(BB_NODEBASE, int);
+    sa.s = {st.StopSplittingThreshold, st.MaxLeafTriangleCount, st.TriangleCost, st.StackOptThreshold, st.StackOptSahIncreaseAcceptance, st.SplitFactor};
+    sa.small = BB_P(BB_SMALL, idkbb::Task); sa.smallCount = counters + 2;
+    idkbb::Task* lists[2] = {BB_P(BB_TASKS0, idkbb::Task), BB_P(BB_TASKS1, idkbb::Task)};
+    sa.in = nullptr; sa.inCount = 0; sa.outBig = lists[0]; sa.outBigCount = counters + 0;
+    k_bb_init_roots<<<(B + 127) / 128, 128, 0, s>>>(sa, BB_P(BB_FRAGCOUNT, int), B);
+    for (int level = 0;; level++) {
+        const int cur = level & 1;
+        int bigCount = 0;
+        CK(cudaMemcpyAsync(&bigCount, counters + cur, 4, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        if (bigCount == 0) break;
+        sa.in = lists[cur]; sa.inCount = bigCount;
+        sa.outBig = lists[cur ^ 1]; sa.outBigCount = counters + (cur ^ 1);
+        CK(cudaMemsetAsync(counters + (cur ^ 1), 0, 4, s));
+        idkbb::k_split_big<<<bigCount, idkbb::NT, 0, s>>>(sa);
+    }
+    int smallCount = 0;
+    CK(cudaMemcpyAsync(&smallCount, counters + 2, 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    if (smallCount) idkbb::k_split_small<<<(smallCount + 63) / 64, 64, 0, s>>>(sa, smallCount);
+    cudaEventRecord(ev[3], s);
+
+    // ---- stack optimisation
+    BB_NEED(BB_PERBLAS, (size_t)B * 64);
+    BB_NEED(BB_NODEI0, ((size_t)NS + 1) * 4); BB_NEED(BB_NODEI1, ((size_t)NS + 1) * 4); BB_NEED(BB_NODEI2, ((size_t)NS + 1) * 4);
+    BB_NEED(BB_NODEI3, ((size_t)NS + 1) * 4 * 8); BB_NEED(BB_NODED0, ((size_t)NS + 1) * 8); BB_NEED(BB_NODED1, ((size_t)NS + 1) * 8 * 2);
+    BB_NEED(BB_TRIOUT, (size_t)F * 16);
+    int* perBlas = BB_P(BB_PERBLAS, int);      // 16 ints per BLAS slot group, laid out as arrays of B
+    CK(cudaMemsetAsync(perBlas, 0, (size_t)B * 64, s));
+    int* nodeI3 = BB_P(BB_NODEI3, int);
+    const size_t NS1 = (size_t)NS + 1;
+    idkbb::PostArgs q;
+    q.nodes = sa.nodes; q.out = BB_P(BB_OUT, GpuBlasNode);
+    q.depth = sa.depth; q.parent = sa.parent; q.rangeStart = sa.rangeStart; q.rangeCount = sa.rangeCount;
+    q.nodeBase = sa.nodeBase; q.fragOffset = sa.fragOffset; q.fragCount = BB_P(BB_FRAGCOUNT, int);
+    q.blasCount = B; q.nodeSlots = NS; q.s = sa.s;
+    q.rootWasLeaf = perBlas; q.created = perBlas + B; q.rs0 = perBlas + 2 * B; q.finalK = perBlas + 3 * B; q.rsOut = perBlas + 4 * B;
+    q.newCount = perBlas + 5 * B; q.triOutCount = perBlas + 6 * B; q.sah = (double*)(perBlas + 8 * B);
+    q.keys = keys; q.vals = vals;
+    q.pre = BB_P(BB_NODEI0, int); q.byDepth = BB_P(BB_NODEI1, int); q.prePos = BB_P(BB_NODEI2, int);
+    q.cflag = nodeI3; q.size = nodeI3 + NS1; q.diff = nodeI3 + 2 * NS1; q.qualPre = nodeI3 + 3 * NS1; q.depthPre = nodeI3 + 4 * NS1;
+    q.internalDep = nodeI3 + 5 * NS1; q.depthDep = nodeI3 + 6 * NS1; q.flag = nodeI3 + 7 * NS1;
+    q.sahPre = BB_P(BB_NODED0, double); q.collPre = BB_P(BB_NODED1, double); q.collDep = q.collPre + NS1;
+    q.newId = q.size;                 // sizes are dead once the stack optimisation has run
+    q.pairCount = q.internalDep; q.uniqCount = q.depthDep; q.uniq = sa.aux;
+    q.sorted0 = sorted[0]; q.fragTri = fa.fragTri; q.tris = pa.tris; q.triOut = BB_P(BB_TRIOUT, int4); q.presplit = pa.blasPresplit;
+    const int nsBlocks = (NS + 256) / 256, bBlocks = (B + 127) / 128;
+    const int nodeEndBit = 48 + bits_for((uint64_t)(B - 1));
+    idkbb::k_root_fix<<<bBlocks, 128, 0, s>>>(q);
+    idkbb::k_node_keys<<<nsBlocks, 256, 0, s>>>(q, 0);
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, tempBytes, keys, keys2, vals, q.pre, NS, 0, nodeEndBit, s));
+    CK(temp(std::max(tempBytes, buf[BB_TEMP].bytes)));
+    tempBytes = buf[BB_TEMP].bytes;
+    CK(cub::DeviceRadixSort::SortPairs(buf[BB_TEMP].p, tempBytes, keys, keys2, vals, q.pre, NS, 0, nodeEndBit, s));
+    idkbb::k_pre_pos<<<nsBlocks, 256, 0, s>>>(q);
+    size_t scanBytes = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, scanBytes, q.cflag, q.cflag, NS + 1, s));
+    size_t incBytes = 0;
+    CK(cub::DeviceScan::InclusiveSum(nullptr, incBytes, q.diff, q.diff, NS + 1, s));
+    CK(temp(std::max(std::max(scanBytes, incBytes), buf[BB_TEMP].bytes)));
+    tempBytes = buf[BB_TEMP].bytes;
+    size_t tb = tempBytes;
+    CK(cub::DeviceScan::ExclusiveSum(buf[BB_TEMP].p, tb, q.cflag, q.cflag, NS + 1, s));
+    idkbb::k_sizes_both<<<nsBlocks, 256, 0, s>>>(q);
+    tb = tempBytes;
+    CK(cub::DeviceScan::InclusiveSum(buf[BB_TEMP].p, tb, q.diff, q.diff, NS + 1, s));
+    idkbb::k_terms<<<nsBlocks, 256, 0, s>>>(q);
+    idkbb::k_node_keys<<<nsBlocks, 256, 0, s>>>(q, 1);
+    tb = tempBytes;
+    CK(cub::DeviceRadixSort::SortPairs(buf[BB_TEMP].p, tb, keys, keys2, vals, q.byDepth, NS, 0, nodeEndBit, s));
+    idkbb::k_dep_arrays<<<nsBlocks, 256, 0, s>>>(q);
+    idkbb::k_stack_opt<<<B, 32, 0, s>>>(q);
+    cudaEventRecord(ev[4], s);
+
+    // ---- compaction (RemoveEmptySubtrees)
+    CK(cudaMemsetAsync(q.out, 0, (size_t)NS * 32, s));
+    idkbb::k_survivors<<<nsBlocks, 256, 0, s>>>(q);
+    tb = tempBytes;
+    CK(cub::DeviceScan::ExclusiveSum(buf[BB_TEMP].p, tb, q.flag, q.flag, NS + 1, s));
+    idkbb::k_emit<<<nsBlocks, 256, 0, s>>>(q);
+    cudaEventRecord(ev[5], s);
+
+    // ---- unindexing, SAH of the result
+    idkbb::k_pair_counts<<<nsBlocks, 256, 0, s>>>(q);
+    idkbb::k_leaf_counts<<<nsBlocks, 256, 0, s>>>(q);
+    tb = tempBytes;
+    CK(cub::DeviceScan::ExclusiveSum(buf[BB_TEMP].p, tb, q.flag, q.flag, NS + 1, s));
+    idkbb::k_unindex_plain<<<nsBlocks, 256, 0, s>>>(q);
+    idkbb::k_unindex_pairs<<<nsBlocks, 256, 0, s>>>(q);
+    idkbb::k_final_terms<<<nsBlocks, 256, 0, s>>>(q);
+    idkbb::k_final_sah<<<B, 32, 0, s>>>(q);
+    cudaEventRecord(ev[6], s);
+    std::vector<int> hostPer((size_t)B * 16);
+    CK(cudaMemcpyAsync(hostPer.data(), perBlas, (size_t)B * 64, cudaMemcpyDeviceToHost, s));
+    cudaError_t e = cudaStreamSynchronize(s);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) { ctx->lastError = std::string("idkpt_blas_build: ") + cudaGetErrorString(e); return IDKPT_ERR_CUDA; }
+    for (int i = 0; i < 6; i++) cudaEventElapsedTime(&bb.phaseMs[i], ev[i], ev[i + 1]);
+    if (kernelMs) cudaEventElapsedTime(kernelMs, ev[0], ev[6]);
+    const double* sah = (const double*)(hostPer.data() + 8 * B);
+    bb.infos.resize(B);
+    for (int b = 0; b < B; b++) {
+        IdkPtBlasBuildInfo& in = bb.infos[b];
+        in.NodeCount = (uint32_t)hostPer[5 * B + b];
+        in.TriangleCount = presplit[b] ? (uint32_t)hostPer[6 * B + b] : (uint32_t)fragCount[b];
+        in.FragmentCount = (uint32_t)fragCount[b];
+        in.RequiredStackSize = hostPer[4 * B + b];
+        memcpy(&in.SahBits, &sah[b], 8);
+        infosOut[b] = in;
+    }
+    bb.nodeBase = nodeBase;
+    bb.fragOffset = fragOff;
+#undef BB_NEED
+#undef BB_P
+    return IDKPT_OK;
+}
+
+IDKPT_API int idkpt_blas_build_read(IdkPtCtx* ctx, uint32_t blas, GpuBlasNode* nodesOut, GpuBlasTriangle* trianglesOut) {
+    if (!ctx) return IDKPT_ERR_INVALID_ARGUMENT;
+    auto& bb = ctx->bb;
+    if (blas >= bb.infos.size()) return fail(ctx, IDKPT_ERR_INVALID_ARGUMENT, "idkpt_blas_build_read: no such BLAS in the last build");
+    CK(cudaSetDevice(ctx->device));
+    const IdkPtBlasBuildInfo& in = bb.infos[blas];
+    if (nodesOut) CK(cudaMemcpyAsync(nodesOut, (const GpuBlasNode*)bb.buf[BB_OUT].p + bb.nodeBase[blas], (size_t)in.NodeCount * 32, cudaMemcpyDeviceToHost, bb.stream));
+    if (trianglesOut) CK(cudaMemcpyAsync(trianglesOut, (const GpuBlasTriangle*)bb.buf[BB_TRIOUT].p + bb.fragOffset[blas], (size_t)in.TriangleCount * 16, cudaMemcpyDeviceToHost, bb.stream));
+    CK(cudaStreamSynchronize(bb.stream));
+    return IDKPT_OK;
+}
+
+IDKPT_API int idkpt_blas_build_phase_ms(IdkPtCtx* ctx, float* phaseMs, int32_t count) {
+    if (!ctx || (!phaseMs && count > 0)) return IDKPT_ERR_INVALID_ARGUMENT;
+    for (int i = 0; i < count && i < 6; i++) phaseMs[i] = ctx->bb.phaseMs[i];
+    return IDKPT_OK;
 }
 
 } // extern "C"

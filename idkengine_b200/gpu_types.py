@@ -43,12 +43,19 @@ IdkPtGpuSettings = np.dtype([("FocalLength", f4), ("LenseRadius", f4), ("DoDebug
 IdkPtRay = np.dtype([("Origin", f4, 3), ("TMax", f4), ("Direction", f4, 3), ("_pad0", f4)])
 IdkPtHit = np.dtype([("BaryX", f4), ("BaryY", f4), ("T", f4), ("TriangleId", u4), ("MeshTransformId", u4),
                      ("NodePairFetches", u4), ("TriangleTests", u4), ("_pad0", u4)])
+IdkPtBlasBuildSettings = np.dtype([("StopSplittingThreshold", i4), ("MaxLeafTriangleCount", i4), ("TriangleCost", f4),
+                                   ("StackOptThreshold", i4), ("StackOptSahIncreaseAcceptance", f4), ("SplitFactor", f4),
+                                   ("DoPreSplit", i4)])
+IdkPtBlasBuildDesc = np.dtype([("TriangleOffset", u4), ("TriangleCount", u4), ("IsRefittable", i4), ("_pad0", i4)])
+IdkPtBlasBuildInfo = np.dtype([("NodeCount", u4), ("TriangleCount", u4), ("FragmentCount", u4), ("RequiredStackSize", i4),
+                               ("SahBits", u8)])
 
 EXPECTED_SIZES = {
     "GpuBlasNode": 32, "GpuBlasTriangle": 16, "GpuBlasDesc": 40, "GpuBlasInstance": 8, "GpuTlasNode": 32,
     "GpuMeshTransform": 144, "GpuMesh": 96, "GpuMaterial": 96, "GpuVertex": 16, "PackedVec3": 12,
     "GpuLight": 48, "GpuPerFrameData": 544, "GpuWavefrontRay": 48, "GpuAovRay": 32, "IdkPtGpuSettings": 20,
     "IdkPtRay": 32, "IdkPtHit": 32, "GpuUnskinnedVertex": 52, "IdkPtSkinningCmd": 16,
+    "IdkPtBlasBuildSettings": 28, "IdkPtBlasBuildDesc": 16, "IdkPtBlasBuildInfo": 24,
 }
 for _name, _size in EXPECTED_SIZES.items():
     assert globals()[_name].itemsize == _size, (_name, globals()[_name].itemsize, _size)

@@ -252,10 +252,13 @@ class Scene:
         self.source_triangle_count = 0
         self.build_info = []
 
-    def add(self, *models, threads=None, cache_dir=None):
+    def add(self, *models, threads=None, cache_dir=None, builder=None):
         """ModelManager.Add (SRC/ModelManager.cs:128-213) + BVH.Add/BlasesBuild (SRC/Bvh/BVH.cs:236-276,300-451):
-        one BLAS + one instance per model. cache_dir (or $IDKHOST_BVH_CACHE): directory of the on-disk BLAS cache."""
+        one BLAS + one instance per model. cache_dir (or $IDKHOST_BVH_CACHE): directory of the on-disk BLAS cache.
+        builder: a callable with build_blas's signature (default: build_blas, the host builder); when it has a `batch`
+        attribute (PathTracer.BlasBuilder), every model of this call that the cache does not hold is built in one batch."""
         cache_dir = cache_dir or os.environ.get("IDKHOST_BVH_CACHE") or None
+        pending = []
         for m in models:
             v_off = len(self.positions)
             mesh_off = len(self.meshes)
@@ -288,7 +291,7 @@ class Scene:
             self.source_triangle_count += len(src)
 
             b = None
-            cache_path = None
+            key = cache_path = None
             if cache_dir is not None:     # skip the SweepSAH build when this exact model was built before
                 key = blas_source_key(m.positions, m.indices, m.tri_mesh, not m.refittable)
                 cache_path = os.path.join(cache_dir, f"{key:016x}.idkbvh")
@@ -298,16 +301,28 @@ class Scene:
                         b["triangles"][f] += v_off
                     b["triangles"]["MeshId"] += mesh_off
                     b["from_cache"] = True
-            if b is None:
-                b = build_blas(self.positions, src, presplit=not m.refittable, threads=threads)
-                if cache_path is not None:
-                    rel = dict(b)
-                    rel["triangles"] = b["triangles"].copy()
-                    for f in ("X", "Y", "Z"):
-                        rel["triangles"][f] -= v_off
-                    rel["triangles"]["MeshId"] -= mesh_off
-                    os.makedirs(cache_dir, exist_ok=True)
-                    cache_save(cache_path, key, rel)
+            pending.append(dict(m=m, src=src, b=b, key=key, cache_path=cache_path, v_off=v_off, mesh_off=mesh_off,
+                                transform_id=transform_id))
+
+        todo = [p for p in pending if p["b"] is None]
+        if todo and builder is not None and getattr(builder, "batch", None) is not None:
+            for p, b in zip(todo, builder.batch(self.positions, [(p["src"], not p["m"].refittable) for p in todo])):
+                p["b"] = b
+        for p in todo:
+            if p["b"] is None:
+                p["b"] = (builder or build_blas)(self.positions, p["src"], presplit=not p["m"].refittable, threads=threads)
+            if p["cache_path"] is not None:
+                b = p["b"]
+                rel = dict(b)
+                rel["triangles"] = b["triangles"].copy()
+                for f in ("X", "Y", "Z"):
+                    rel["triangles"][f] -= p["v_off"]
+                rel["triangles"]["MeshId"] -= p["mesh_off"]
+                os.makedirs(cache_dir, exist_ok=True)
+                cache_save(p["cache_path"], p["key"], rel)
+
+        for p in pending:
+            m, b, src = p["m"], p["b"], p["src"]
             desc = np.zeros(1, gt.GpuBlasDesc)
             desc["NodeOffset"] = len(self.blas_nodes)
             desc["NodeCount"] = len(b["nodes"])
@@ -321,7 +336,7 @@ class Scene:
             self.blas_triangles = np.concatenate([self.blas_triangles, b["triangles"]])
             inst = np.zeros(1, gt.GpuBlasInstance)
             inst["BlasId"] = blas_id
-            inst["MeshTransformId"] = transform_id
+            inst["MeshTransformId"] = p["transform_id"]
             self.blas_instances = np.concatenate([self.blas_instances, inst])
             self.build_info.append(dict(name=m.name, source_triangles=len(src), fragments=b["fragment_count"],
                                         triangles=len(b["triangles"]), nodes=len(b["nodes"]),

@@ -33,6 +33,7 @@
 #include <string>
 
 #include "../../include/idk_gpu_types.h"
+#include "../../include/idk_cbrtf.h"
 
 namespace {
 
@@ -162,7 +163,7 @@ static float priority(const Tri& t) {
     V3 c = cross(t.p1 - t.p0, t.p2 - t.p0);
     float triArea = sqrtf(c.x * c.x + c.y * c.y + c.z * c.z) * 0.5f;
     float emptyAreaPrio = b.area() - triArea;
-    return cbrtf(extentPrio * emptyAreaPrio);
+    return idk_cbrtf(extentPrio * emptyAreaPrio);   // glibc's cbrtf, restated: include/idk_cbrtf.h
 }
 
 static int getSplitCount(float prio, float totalPrio, int triCount, float splitFactor) {
@@ -796,7 +797,9 @@ static void unindexPlain(BuildResult& blas, const BuildData& bd, const Geometry&
     for (size_t i = 2; i < blas.nodes.size(); i++) {
         GpuBlasNode& n = blas.nodes[i];
         if (n.TriCount > 0) {
-            for (int j = 0; j < n.TriCount; j++) tris[counter + j] = g.tris[bd.sorted[0][n.TriStartOrChild + j]];
+            // A root that did not split is listed twice (nodes 2 and 3); the second copy's triangles fall past the
+            // array's end and are dropped rather than written out of bounds.
+            for (int j = 0; j < n.TriCount && counter + j < (int)tris.size(); j++) tris[counter + j] = g.tris[bd.sorted[0][n.TriStartOrChild + j]];
             n.TriStartOrChild = counter;
             counter += n.TriCount;
         }
@@ -911,6 +914,12 @@ void idkhost_blas_copy(const IdkBlasBuild* b, GpuBlasNode* nodes, GpuBlasTriangl
     memcpy(tris, b->tris.data(), b->tris.size() * sizeof(GpuBlasTriangle));
 }
 __attribute__((visibility("default"))) void idkhost_blas_free(IdkBlasBuild* b) { delete b; }
+
+// The builder's cube root (include/idk_cbrtf.h) over an array, for tests that compare it with the C library.
+__attribute__((visibility("default")))
+void idkhost_cbrtf(const float* x, float* out, uint64_t count) {
+    for (uint64_t i = 0; i < count; i++) out[i] = idk_cbrtf(x[i]);
+}
 
 } // extern "C"
 

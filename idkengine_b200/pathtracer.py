@@ -139,6 +139,63 @@ class PathTracer:
         self._check(self._lib.idkpt_tlas_build(self._ctx, search_radius, ctypes.byref(ms)), "idkpt_tlas_build")
         return ms.value
 
+    def BuildBlases(self, positions, jobs, settings=None):
+        """BVH.BlasesBuild (BVH.cs:300-377) on the device, every BLAS of the batch in one call. positions: PackedVec3[V];
+        jobs: list of (triangles: GpuBlasTriangle[T] with global vertex ids, presplit). settings: host.IdkBlasBuildSettings
+        or capi.IdkPtBlasBuildSettings (Threads and DoPreSplit are ignored; presplit decides). Returns one dict per job,
+        equal to what host.build_blas returns for the same input."""
+        positions = np.ascontiguousarray(positions)
+        assert positions.dtype == gt.PackedVec3
+        tris = [np.ascontiguousarray(t) for t, _ in jobs]
+        assert all(t.dtype == gt.GpuBlasTriangle for t in tris)
+        allt = np.concatenate(tris) if tris else np.zeros(0, gt.GpuBlasTriangle)
+        descs = np.zeros(len(jobs), gt.IdkPtBlasBuildDesc)
+        descs["TriangleCount"] = [len(t) for t in tris]
+        descs["TriangleOffset"] = np.concatenate([[0], np.cumsum(descs["TriangleCount"])[:-1]]) if len(jobs) else []
+        descs["IsRefittable"] = [0 if presplit else 1 for _, presplit in jobs]
+        st = capi.IdkPtBlasBuildSettings()
+        self._lib.idkpt_blas_default_build_settings(ctypes.byref(st))
+        if settings is not None:
+            for name, _ in capi.IdkPtBlasBuildSettings._fields_:
+                if name != "DoPreSplit":
+                    setattr(st, name, getattr(settings, name))
+        st.DoPreSplit = 1
+        infos = np.zeros(len(jobs), gt.IdkPtBlasBuildInfo)
+        ms = ctypes.c_float()
+        self._check(self._lib.idkpt_blas_build(self._ctx, positions.ctypes.data, len(positions), allt.ctypes.data if len(allt) else None,
+                                               len(allt), descs.ctypes.data, len(jobs), ctypes.byref(st), infos.ctypes.data,
+                                               ctypes.byref(ms)), "idkpt_blas_build")
+        self.last_blas_build_ms = ms.value
+        out = []
+        for b, info in enumerate(infos):
+            nodes = np.zeros(int(info["NodeCount"]), gt.GpuBlasNode)
+            tri = np.zeros(int(info["TriangleCount"]), gt.GpuBlasTriangle)
+            self._check(self._lib.idkpt_blas_build_read(self._ctx, b, nodes.ctypes.data, tri.ctypes.data), "idkpt_blas_build_read")
+            out.append(dict(nodes=nodes, triangles=tri, required_stack_size=int(info["RequiredStackSize"]),
+                            fragment_count=int(info["FragmentCount"]), sah=float(np.array(info["SahBits"], np.uint64).view(np.float64))))
+        return out
+
+    def BuildBlas(self, positions, triangles, presplit=True, settings=None, threads=None):
+        """One BLAS on the device: the same dict as host.build_blas(positions, triangles, presplit, settings=settings).
+        threads is accepted for signature compatibility and ignored."""
+        return self.BuildBlases(positions, [(triangles, presplit)], settings)[0]
+
+    @property
+    def BlasBuilder(self):
+        """A builder for host.Scene.add(builder=...): called like host.build_blas, with .batch building all models of one add()."""
+        pt = self
+
+        def build(positions, triangles, presplit=True, threads=None, settings=None):
+            return pt.BuildBlas(positions, triangles, presplit, settings)
+        build.batch = lambda positions, jobs, settings=None: pt.BuildBlases(positions, jobs, settings)
+        return build
+
+    def BlasBuildPhaseMs(self):
+        """Device ms of the last build: pre-split, sort, splits, stack optimisation, compaction, unindexing."""
+        ms = (ctypes.c_float * 6)()
+        self._check(self._lib.idkpt_blas_build_phase_ms(self._ctx, ms, 6), "idkpt_blas_build_phase_ms")
+        return dict(zip(("presplit", "sort", "splits", "stack_opt", "compaction", "unindex"), list(ms)))
+
     def SetTextures(self, textures):
         """Replace the material texture table (list of dict(pixels, srgb, wrap_s, wrap_t), as host.Scene.textures)."""
         arr, keep = capi.texture_descs(textures)

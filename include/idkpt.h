@@ -313,6 +313,54 @@ IDKPT_API int idkpt_read_range(IdkPtCtx* ctx, IdkPtArrayId which, uint64_t first
  * scene's TLAS node array (UseTlas scenes) with exactly the nodes the host build produces -- a moving scene reads nothing back. */
 IDKPT_API int idkpt_tlas_build(IdkPtCtx* ctx, int32_t search_radius, float* kernel_ms);
 
+/* ---- BLAS build on the device (SURVEY.md 8f row 4): BVH.BlasesBuild(start, count) (BVH.cs:300-377) for a batch of BLASes.
+ * SweepSAH with pre-splitting, node for node and byte for byte equal to the host builder (host_mirror/bvh_build.cpp, the
+ * C# BLAS.Build it mirrors). A pure function of its inputs: it reads and writes no scene, image or accumulation state and
+ * works on a context without a scene. Results live in the context until the next build or idkpt_destroy.
+ *   positions: PackedVec3[positionCount]; triangles: GpuBlasTriangle[triangleCount] with global vertex ids and MeshId set
+ *   (what BVH.Add produces); descs[blasCount]: one BLAS each, over triangles[TriangleOffset, TriangleOffset + TriangleCount).
+ *   settings: NULL = idkpt_blas_default_build_settings. infos_out[blasCount] receives each BLAS's sizes.
+ * IDKPT_ERR_INVALID_ARGUMENT: a vertex index outside positionCount, an empty BLAS, a range outside the triangle array,
+ *   a non-finite position, or a BLAS whose bounding box has a non-finite half-area (NaN split costs).
+ * IDKPT_ERR_UNSUPPORTED: a BLAS of 2^24 fragments or more (the builder counts in floats), more than 65535 BLASes or
+ *   2^31 fragments in one call. */
+typedef struct IdkPtBlasBuildSettings {   /* BLAS.BuildSettings (BLAS.cs:31-48) + PreSplitting.Settings (PreSplitting.cs:17-24) */
+    int32_t StopSplittingThreshold;       /* 1 */
+    int32_t MaxLeafTriangleCount;         /* 2 */
+    float   TriangleCost;                 /* 1.1 */
+    int32_t StackOptThreshold;            /* 16 */
+    float   StackOptSahIncreaseAcceptance;/* 0.0009745 */
+    float   SplitFactor;                  /* 0.3 */
+    int32_t DoPreSplit;                   /* 1: pre-split every BLAS whose IsRefittable is 0 */
+} IdkPtBlasBuildSettings;
+IDK_STATIC_ASSERT(sizeof(IdkPtBlasBuildSettings) == 28, "IdkPtBlasBuildSettings must be 28 bytes");
+
+typedef struct IdkPtBlasBuildDesc {
+    uint32_t TriangleOffset;              /* into the call's triangle array */
+    uint32_t TriangleCount;
+    int32_t  IsRefittable;                /* 0 selects pre-splitting (BVH.cs:324-333) */
+    int32_t  _pad0;
+} IdkPtBlasBuildDesc;
+IDK_STATIC_ASSERT(sizeof(IdkPtBlasBuildDesc) == 16, "IdkPtBlasBuildDesc must be 16 bytes");
+
+typedef struct IdkPtBlasBuildInfo {       /* what the host builder reports for the same BLAS */
+    uint32_t NodeCount;                   /* GpuBlasNode records, node 0 = pad, node 1 = root */
+    uint32_t TriangleCount;               /* GpuBlasTriangle records (unindexed) */
+    uint32_t FragmentCount;               /* triangles after pre-splitting */
+    int32_t  RequiredStackSize;
+    uint64_t SahBits;                     /* BLAS.ComputeGlobalSAH of the result: the bits of the double (memcpy / BitConverter) */
+} IdkPtBlasBuildInfo;
+IDK_STATIC_ASSERT(sizeof(IdkPtBlasBuildInfo) == 24, "IdkPtBlasBuildInfo must be 24 bytes");
+
+IDKPT_API void idkpt_blas_default_build_settings(IdkPtBlasBuildSettings* settings);
+IDKPT_API int idkpt_blas_build(IdkPtCtx* ctx, const PackedVec3* positions, uint64_t positionCount, const GpuBlasTriangle* triangles,
+                               uint64_t triangleCount, const IdkPtBlasBuildDesc* descs, uint32_t blasCount,
+                               const IdkPtBlasBuildSettings* settings, IdkPtBlasBuildInfo* infos_out, float* kernel_ms);
+/* Copies BLAS `blas` of the last build: nodes_out[NodeCount], triangles_out[TriangleCount] (either may be NULL). */
+IDKPT_API int idkpt_blas_build_read(IdkPtCtx* ctx, uint32_t blas, GpuBlasNode* nodes_out, GpuBlasTriangle* triangles_out);
+/* Device time of the last build's phases in ms: pre-split, sort, splits, stack optimisation, compaction, unindexing. */
+IDKPT_API int idkpt_blas_build_phase_ms(IdkPtCtx* ctx, float* phase_ms_out, int32_t count);
+
 /* ---- present chain (SURVEY.md 8f.3): Bloom.Compute(Result) + TonemapAndGamma.Compute(Result, Bloom.Result)
  * (Application.cs:217-223) -> the RGBA8 frame the reference copies to the swapchain, produced on the device. ---- */
 typedef struct IdkPtPostSettings {

@@ -54,6 +54,15 @@ with PathTracer(64, 48) as pt:
     pt.Compute()
 print("dynamic ok")
 
+# device BLAS build: a pre-split and a refittable BLAS in one batch, a single-triangle BLAS, read back
+with PathTracer(16, 16) as pt:
+    rng = np.random.default_rng(6)
+    pts = np.zeros(900, gt.PackedVec3)
+    for c in "xyz": pts[c] = rng.uniform(-1, 1, 900).astype(np.float32)
+    t = np.zeros(300, gt.GpuBlasTriangle); t["X"], t["Y"], t["Z"] = np.arange(0, 900, 3), np.arange(1, 900, 3), np.arange(2, 900, 3)
+    pt.BuildBlases(pts, [(t[:200], True), (t[200:299], False), (t[299:], True)])
+print("blas build ok")
+
 # round 2 additions: TLAS walk inside k_traverse2 (async lanes), BC7 / BC5 / BC4 decode at upload, float textures, cube-map sky
 # with seamless filtering, denoise hand-off, point-shadowed lights in the voxeliser
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests"))
